@@ -301,6 +301,46 @@ def states_digest(ss, first=0, count=None):
     return h.hexdigest()[:16]
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, codec, ss, x_dev, out_dev, digest):
+    """Writes what the last timed step handed its caller, as DIR/<name>.npy, so that two builds can be compared output
+    for output:
+      pixels   float32 [n, C, H, W]  the decoded images of the last step (still in out_dev)
+      words    float64 [sum]         each stream's trimmed bitstream (the words above the lowest depth it reached), concatenated
+      lengths  float64 [n]           words per stream in `words`
+      base     float64 [n]           that lowest depth: the seed words below it are not part of the bitstream
+      heads    float64 [n, 2]        the 64-bit ANS heads as (low, high) 32-bit halves
+      streams  float64 [n]           which streams these are
+    The step's decode consumed the bitstreams its encode produced, so they are produced again here, outside the timed
+    region, by encoding the same images onto the same initial states; their digest must equal that of the untimed first
+    encode, i.e. every step coded the same words.  n is every stream unless 64 MB cannot hold them (bounded by the stream
+    capacity, so n depends on the arguments only); then it is a fixed seeded sample."""
+    B = ss.n
+    pixels = out_dev.cpu().numpy()
+    codec.encode(ss, x_dev)
+    torch.cuda.synchronize()
+    ss.raise_on_error()
+    assert states_digest(ss) == digest, "the re-encoded streams differ from the first encode of the same images"
+    words, offs, heads, base = (a.copy() for a in ss.export_packed(trim=True))
+    codec.decode(ss, B, out=out_dev)
+    torch.cuda.synchronize()
+    ss.raise_on_error()
+    assert torch.equal(out_dev, x_dev), "round trip failed"
+    n = min(B, DUMP_BYTES // (8 * ss.capacity + 8 * 5 + 4 * pixels[0].size))
+    idx = np.arange(B) if n == B else np.sort(np.random.RandomState(0).choice(B, n, replace=False))
+    arrays = {"pixels": pixels[idx].astype(np.float32),
+              "words": np.concatenate([words[offs[i]:offs[i + 1]] for i in idx]).astype(np.float64),
+              "lengths": np.diff(offs)[idx].astype(np.float64),
+              "base": base[idx].astype(np.float64),
+              "heads": np.stack([heads[idx] & 0xffffffff, heads[idx] >> 32], axis=1).astype(np.float64),
+              "streams": idx.astype(np.float64)}
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -321,7 +361,11 @@ def main():
     ap.add_argument("--fused-coder", action="store_true", help="one-warp-per-stream fused coder kernels instead of the two-phase coder")
     ap.add_argument("--crop-images", type=int, default=100)
     ap.add_argument("--hwc-quirk", action="store_true", help="crop: feed blocks as imagenetcrop_compress.py:130 does")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the pixels and bitstreams of the last step "
+                    "as DIR/<name>.npy (float32/float64, at most 64 MB; rank 0's streams)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.config == "crop"):
+        ap.error("--dump-outputs writes the outputs of the GPU arm's per-image configurations (not --impl reference or --config crop)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -436,6 +480,8 @@ def main():
     gat_ms = sum(ev[3 * i + 1].elapsed_time(ev[3 * i + 2]) for i in range(args.steps))
     dec_ms = sum(ev[3 * i + 2].elapsed_time(ev[3 * i + 3]) for i in range(args.steps))
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, codec, ss, x_dev, out_dev, digest)
     gather_info = None
     if world > 1:
         gathered_words = int(counts[:, 0].sum())
