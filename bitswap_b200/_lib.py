@@ -135,6 +135,8 @@ def _set_argtypes(L):
         "bsw_codec_destroy": [P],
         "bsw_codec_encode": [P, P, I, I, P, I, P],
         "bsw_codec_decode": [P, P, I, I, P, I, P],
+        "bsw_codec_encode_ext": [P, P, I, I, P, P, I, P],
+        "bsw_codec_decode_ext": [P, P, I, I, P, P, I, P],
         "bsw_codec_last_launches": [P],
         "bsw_codec_profile": [P, I, P, P],
         "bsw_codec_set_two_phase": [P, I],
@@ -160,7 +162,7 @@ EXPORTS = ["bsw_last_error", "bsw_version", "bsw_has_tensor_cores", "bsw_measure
            "bsw_bins_destroy", "bsw_bins_device_ptrs", "bsw_gather_zcentres", "bsw_gather_xcentres",
            "bsw_model_create", "bsw_model_destroy", "bsw_model_load_conv", "bsw_model_load_gen_std",
            "bsw_model_finalize", "bsw_vae_infer", "bsw_vae_generate", "bsw_codec_create", "bsw_codec_destroy",
-           "bsw_codec_encode", "bsw_codec_decode", "bsw_codec_last_launches", "bsw_codec_profile", "bsw_codec_set_two_phase", "bsw_codec_set_dual_stream",
+           "bsw_codec_encode", "bsw_codec_decode", "bsw_codec_encode_ext", "bsw_codec_decode_ext", "bsw_codec_last_launches", "bsw_codec_profile", "bsw_codec_set_two_phase", "bsw_codec_set_dual_stream",
            "bsw_discretize_reset", "bsw_discretize_sample", "bsw_discretize_fold", "bsw_discretize_edges"]
 
 

@@ -68,28 +68,52 @@ class BitSwapCodec:
                 pass
             self._h = None
 
-    def encode(self, streams: StreamSet, x: torch.Tensor, first=0, scheme=BITSWAP):
-        """x: uint8 CUDA tensor [count, C, 32, 32]; pushes one image onto each of `count` streams. Async."""
+    def encode(self, streams: StreamSet, x: torch.Tensor, first=0, scheme=BITSWAP, extents=None):
+        """x: uint8 CUDA tensor [count, C, 32, 32]; pushes one image onto each of `count` streams. Async.
+
+        extents: None (whole blocks) or a contiguous int32 CUDA tensor [count, 2] of (valid_rows, valid_cols), each in
+        [1, 32]: partial blocks.  Only pixels (y, x) with y < valid_rows and x < valid_cols are coded; the others are
+        replaced by the edge-replicate fill before the nets see the block.  An extent outside [1, 32] flags its stream
+        (StreamSet.raise_on_error) and leaves the other streams alone."""
         assert x.is_cuda and x.dtype == torch.uint8 and x.is_contiguous()
         self._same_device(streams, x)
         count = x.shape[0]
+        ext = self._extents_ptr(extents, count)
         with on_device(self.device):
-            check(lib().bsw_codec_encode(self._h, streams.handle, first, count, x.data_ptr(), scheme, cuda_stream_ptr()))
+            if ext is None:
+                check(lib().bsw_codec_encode(self._h, streams.handle, first, count, x.data_ptr(), scheme, cuda_stream_ptr()))
+            else:
+                check(lib().bsw_codec_encode_ext(self._h, streams.handle, first, count, x.data_ptr(), ext, scheme, cuda_stream_ptr()))
+
+    def _extents_ptr(self, extents, count):
+        if extents is None:
+            return None
+        if not (torch.is_tensor(extents) and extents.is_cuda and extents.dtype == torch.int32 and extents.is_contiguous()
+                and tuple(extents.shape) == (count, 2)):
+            raise ValueError(f"extents: need a contiguous int32 CUDA tensor of shape ({count}, 2)")
+        if extents.device.index != self.device:
+            raise ValueError(f"codec is on cuda:{self.device}; extents on {extents.device}")
+        return extents.data_ptr()
 
     def _same_device(self, streams, x=None):
         if streams.device != self.device or (x is not None and x.device.index != self.device):
             raise ValueError(f"codec is on cuda:{self.device}; streams on cuda:{streams.device}"
                              + (f", pixels on {x.device}" if x is not None else ""))
 
-    def decode(self, streams: StreamSet, count: int, first=0, scheme=BITSWAP, out=None):
-        """Pops one image from each stream; returns uint8 CUDA tensor [count, C, 32, 32]. Async."""
+    def decode(self, streams: StreamSet, count: int, first=0, scheme=BITSWAP, out=None, extents=None):
+        """Pops one image from each stream; returns uint8 CUDA tensor [count, C, 32, 32]. Async.
+        extents: as for encode() (the same values the images were encoded with); masked pixels come back as the fill."""
         if out is None:
             out = torch.empty((count,) + tuple(self.cfg.xs), dtype=torch.uint8, device=torch.device("cuda", self.device))
         if not (out.is_cuda and out.dtype == torch.uint8 and out.is_contiguous() and out.numel() >= count * int(np.prod(self.cfg.xs))):
             raise ValueError("decode(out=...): need a contiguous uint8 CUDA tensor with room for `count` images")
         self._same_device(streams, out)
+        ext = self._extents_ptr(extents, count)
         with on_device(self.device):
-            check(lib().bsw_codec_decode(self._h, streams.handle, first, count, out.data_ptr(), scheme, cuda_stream_ptr()))
+            if ext is None:
+                check(lib().bsw_codec_decode(self._h, streams.handle, first, count, out.data_ptr(), scheme, cuda_stream_ptr()))
+            else:
+                check(lib().bsw_codec_decode_ext(self._h, streams.handle, first, count, out.data_ptr(), ext, scheme, cuda_stream_ptr()))
         return out
 
     @property
@@ -180,14 +204,18 @@ class PipelinedCodec:
         for st in self.streams:
             cur.wait_stream(st)
 
-    def encode(self, streams: StreamSet, x: torch.Tensor, first=0, scheme=BITSWAP):
+    def encode(self, streams: StreamSet, x: torch.Tensor, first=0, scheme=BITSWAP, extents=None):
         assert x.is_cuda and x.dtype == torch.uint8 and x.is_contiguous() and x.shape[0] <= self.max_batch
-        self._fan(x.shape[0], lambda c, b, n: c.encode(streams, x[b:b + n], first=first + b, scheme=scheme))
+        self.codecs[0]._extents_ptr(extents, x.shape[0])          # (shape / dtype / device checked before any lane starts)
+        self._fan(x.shape[0], lambda c, b, n: c.encode(streams, x[b:b + n], first=first + b, scheme=scheme,
+                                                       extents=None if extents is None else extents[b:b + n]))
 
-    def decode(self, streams: StreamSet, count: int, first=0, scheme=BITSWAP, out=None):
+    def decode(self, streams: StreamSet, count: int, first=0, scheme=BITSWAP, out=None, extents=None):
         if out is None:
             out = torch.empty((count,) + tuple(self.cfg.xs), dtype=torch.uint8, device=torch.device("cuda", self.device))
-        self._fan(count, lambda c, b, n: c.decode(streams, n, first=first + b, scheme=scheme, out=out[b:b + n]))
+        self.codecs[0]._extents_ptr(extents, count)
+        self._fan(count, lambda c, b, n: c.decode(streams, n, first=first + b, scheme=scheme, out=out[b:b + n],
+                                                  extents=None if extents is None else extents[b:b + n]))
         return out
 
     def set_two_phase(self, on=True):

@@ -672,10 +672,13 @@ __device__ __forceinline__ void load_tile_row(double (&e)[NB], const double *til
     for (int j = 0; j < NB; ++j) e[j] = tile[lane * (NB + 1) + j];
 }
 
-template <int NB>
+// MASK: rowmask holds L/32 words per stream; a clear bit (i & 31) of word i/32 skips row i (template flag: the unmasked
+// loop is the plain one)
+template <int NB, bool MASK>
 __global__ void __launch_bounds__(FW * 32) k_logistic_pop(bsw_streams sv, int first, int count,
         const float *__restrict__ mu, int64_t mss, const float *__restrict__ sc, int64_t sss,
-        const double *__restrict__ endp, int64_t ers, int16_t *__restrict__ sym, int64_t L, int bits, int q) {
+        const double *__restrict__ endp, int64_t ers, int16_t *__restrict__ sym, int64_t L, int bits, int q,
+        const uint32_t *__restrict__ rowmask) {
     extern __shared__ double smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     int si = blockIdx.x * FW + warp;
@@ -684,6 +687,8 @@ __global__ void __launch_bounds__(FW * 32) k_logistic_pop(bsw_streams sv, int fi
     WarpStream ws;
     ws.open(sv, b);
     if (ws.err) return;
+    const uint32_t *rm = MASK ? rowmask + (int64_t)si * (L >> 5) : nullptr;
+    uint32_t live = FULL;              // row mask word of the current block of 32 rows (NULL mask: every row)
     double *tile0 = smem + (size_t)warp * 2 * tile_doubles<NB>();
     double *tile1 = tile0 + tile_doubles<NB>();
     const float *mub = mu + (int64_t)si * mss, *scb = sc + (int64_t)si * sss;
@@ -704,6 +709,7 @@ __global__ void __launch_bounds__(FW * 32) k_logistic_pop(bsw_streams sv, int fi
             int64_t r = (i & ~(int64_t)31) + lane;
             mu_w = r < L ? mub[r] : 0.f;
             sc_w = r < L ? scb[r] : 1.f;
+            if (MASK) live = __ldg(rm + (i >> 5));
         }
         double *tile = cur ? tile1 : tile0;
         if (!shared_row || i == L - 1) {
@@ -715,6 +721,13 @@ __global__ void __launch_bounds__(FW * 32) k_logistic_pop(bsw_streams sv, int fi
                 cp_async_commit();
                 cur ^= 1;
             }
+        }
+        if (MASK && !((live >> j32) & 1u)) {           // masked row: nothing decoded, the symbol slot keeps what it held
+            if (j32 == 0) {
+                int64_t r = i + lane;
+                if (r < L) sy[r] = (int16_t)my_sym;
+            }
+            continue;
         }
         RowTable<NB> T;
         build_row<NB>(e, __shfl_sync(FULL, mu_w, j32), __shfl_sync(FULL, sc_w, j32), mult, bits, lane, T);
@@ -743,10 +756,11 @@ __global__ void __launch_bounds__(FW * 32) k_logistic_pop(bsw_streams sv, int fi
     ws.close(sv, b, lane);
 }
 
-template <int NB>
+template <int NB, bool MASK>
 __global__ void __launch_bounds__(FW * 32) k_logistic_push(bsw_streams sv, int first, int count,
         const float *__restrict__ mu, int64_t mss, const float *__restrict__ sc, int64_t sss,
-        const double *__restrict__ endp, int64_t ers, const int16_t *__restrict__ sym, int64_t L, int bits, int q) {
+        const double *__restrict__ endp, int64_t ers, const int16_t *__restrict__ sym, int64_t L, int bits, int q,
+        const uint32_t *__restrict__ rowmask) {
     extern __shared__ double smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     int si = blockIdx.x * FW + warp;
@@ -762,12 +776,14 @@ __global__ void __launch_bounds__(FW * 32) k_logistic_push(bsw_streams sv, int f
     const int16_t *sy = sym + (int64_t)si * L;
     const double mult = (double)(((int64_t)1 << bits) - ((int64_t)1 << q));
     const bool shared_row = (ers == 0);
+    const uint32_t *rm = MASK ? rowmask + (int64_t)si * (L >> 5) : nullptr;
 
     double e[NB];
     stage_row<NB>(tile0, endp, lane);
     cp_async_commit();
     float mu_w = 0.f, sc_w = 1.f;
     int sym_w = 0;
+    uint32_t live = FULL;
     int cur = 0;
     for (int64_t i = 0; i < L; ++i) {
         int j32 = (int)(i & 31);
@@ -776,6 +792,7 @@ __global__ void __launch_bounds__(FW * 32) k_logistic_push(bsw_streams sv, int f
             mu_w = r < L ? mub[r] : 0.f;
             sc_w = r < L ? scb[r] : 1.f;
             sym_w = r < L ? (int)sy[r] : 0;
+            if (MASK) live = __ldg(rm + (i >> 5));
         }
         double *tile = cur ? tile1 : tile0;
         if (!shared_row || i == 0) {
@@ -788,6 +805,7 @@ __global__ void __launch_bounds__(FW * 32) k_logistic_push(bsw_streams sv, int f
                 cur ^= 1;
             }
         }
+        if (MASK && !((live >> j32) & 1u)) continue;  // masked row: head and word stack untouched
         RowTable<NB> T;
         build_row<NB>(e, __shfl_sync(FULL, mu_w, j32), __shfl_sync(FULL, sc_w, j32), mult, bits, lane, T);
         int s = __shfl_sync(FULL, sym_w, j32);
@@ -812,33 +830,39 @@ __global__ void __launch_bounds__(FW * 32) k_logistic_push(bsw_streams sv, int f
 template <int NB>
 static int launch_fused(bool push, bsw_streams *s, int first, int count, const float *mu, int64_t mss, const float *sc,
                         int64_t sss, const double *endp, int64_t ers, int16_t *sym, int64_t L, int bits, int q,
-                        cudaStream_t st) {
+                        const uint32_t *rowmask, cudaStream_t st) {
     size_t smem = (size_t)FW * 2 * tile_doubles<NB>() * sizeof(double);
+    const unsigned g = (count + FW - 1) / FW;
+#define FUSED_LAUNCH(K)                                                                                                       \
+    do {                                                                                                                      \
+        BSW_CUDA(cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                            \
+        K<<<g, FW * 32, smem, st>>>(*s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, rowmask);                 \
+    } while (0)
     if (push) {
-        BSW_CUDA(cudaFuncSetAttribute(k_logistic_push<NB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_logistic_push<NB><<<(count + FW - 1) / FW, FW * 32, smem, st>>>(*s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q);
+        if (rowmask) FUSED_LAUNCH((k_logistic_push<NB, true>)); else FUSED_LAUNCH((k_logistic_push<NB, false>));
     } else {
-        BSW_CUDA(cudaFuncSetAttribute(k_logistic_pop<NB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_logistic_pop<NB><<<(count + FW - 1) / FW, FW * 32, smem, st>>>(*s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q);
+        if (rowmask) FUSED_LAUNCH((k_logistic_pop<NB, true>)); else FUSED_LAUNCH((k_logistic_pop<NB, false>));
     }
+#undef FUSED_LAUNCH
     BSW_LAUNCH_CHECK();
     return BSW_OK;
 }
 static int dispatch_fused(bool push, bsw_streams *s, int first, int count, const float *mu, int64_t mss, const float *sc,
                           int64_t sss, const double *endp, int64_t ers, int16_t *sym, int64_t L, int S, int bits, int q,
-                          void *stream) {
+                          const uint32_t *rowmask, void *stream) {
     if (int rc = check_range(s, first, count)) return rc;
     BSW_REQUIRE(mu && sc && endp && sym && L > 0, "fused coder: null argument");
     BSW_REQUIRE(bits > 0 && bits <= 31 && q >= 0 && q < bits, "fused coder: bits/quantbits out of range");
     BSW_REQUIRE((ers == 0 || ers >= S) && (((uintptr_t)endp) & 7) == 0, "fused coder: endpoint rows must hold S doubles (+inf padded)");
+    BSW_REQUIRE(!rowmask || (L & 31) == 0, "fused coder: a row mask needs a multiple of 32 rows");
     cudaStream_t st = (cudaStream_t)stream;
     switch (S) {
-        case 32:   return launch_fused<1>(push, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, st);
-        case 64:   return launch_fused<2>(push, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, st);
-        case 128:  return launch_fused<4>(push, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, st);
-        case 256:  return launch_fused<8>(push, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, st);
-        case 512:  return launch_fused<16>(push, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, st);
-        case 1024: return launch_fused<32>(push, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, st);
+        case 32:   return launch_fused<1>(push, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, rowmask, st);
+        case 64:   return launch_fused<2>(push, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, rowmask, st);
+        case 128:  return launch_fused<4>(push, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, rowmask, st);
+        case 256:  return launch_fused<8>(push, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, rowmask, st);
+        case 512:  return launch_fused<16>(push, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, rowmask, st);
+        case 1024: return launch_fused<32>(push, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, rowmask, st);
     }
     bsw_set_error("fused coder: support must be one of 32,64,...,1024 (got %d)", S);
     return BSW_E_INVALID;
@@ -846,12 +870,19 @@ static int dispatch_fused(bool push, bsw_streams *s, int first, int count, const
 extern "C" int bsw_logistic_push(bsw_streams *s, int first, int count, const float *mu, int64_t mss, const float *sc,
                                  int64_t sss, const double *endp, int64_t ers, const int16_t *sym, int64_t L, int S,
                                  int bits, int q, void *stream) {
-    return dispatch_fused(true, s, first, count, mu, mss, sc, sss, endp, ers, (int16_t *)sym, L, S, bits, q, stream);
+    return dispatch_fused(true, s, first, count, mu, mss, sc, sss, endp, ers, (int16_t *)sym, L, S, bits, q, nullptr, stream);
 }
 extern "C" int bsw_logistic_pop(bsw_streams *s, int first, int count, const float *mu, int64_t mss, const float *sc,
                                 int64_t sss, const double *endp, int64_t ers, int16_t *sym, int64_t L, int S, int bits,
                                 int q, void *stream) {
-    return dispatch_fused(false, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, S, bits, q, stream);
+    return dispatch_fused(false, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, S, bits, q, nullptr, stream);
+}
+// The fused coder with a row mask (NULL = every row; L/32 words per stream, a clear bit (i & 31) of word i/32 skips row i):
+// what the codec calls for the pixel level of a partial block.
+int bsw_logistic_fused(bool pop, bsw_streams *s, int first, int count, const float *mu, int64_t mss, const float *sc,
+                       int64_t sss, const double *endp, int64_t ers, int16_t *sym, int64_t L, int S, int bits, int q,
+                       const uint32_t *rowmask, cudaStream_t st) {
+    return dispatch_fused(!pop, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, S, bits, q, rowmask, st);
 }
 
 // ================================================================================================

@@ -269,8 +269,12 @@ __global__ void __launch_bounds__(RW * 32, 2) k_rows(int count, int64_t L, const
 
 // ---- phase B: push -------------------------------------------------------------------------------------------------
 constexpr int BW = 4;
+// MASK: rowmask holds L/32 words per stream; bit (i & 31) of word si * L/32 + i/32 clear -> row i of stream si is not
+// coded.  (A template flag rather than a NULL test, so that the unmasked kernel is the plain loop: the per-row test cost
+// 16 % of this latency-bound kernel when it was always compiled in.)
+template <bool MASK>
 __global__ void __launch_bounds__(BW * 32) k_push_pairs(bsw_streams sv, int first, int count, const uint4 *__restrict__ pairs,
-                                                        int64_t L, int bits) {
+                                                        int64_t L, int bits, const uint32_t *__restrict__ rowmask) {
     const int lane = threadIdx.x & 31;
     const int si = blockIdx.x * BW + (threadIdx.x >> 5);
     if (si >= count) return;
@@ -280,13 +284,16 @@ __global__ void __launch_bounds__(BW * 32) k_push_pairs(bsw_streams sv, int firs
     if (ws.err) return;
     ws.push_begin(lane);
     const uint4 *pp = pairs + (int64_t)si * L;
+    const uint32_t *rm = MASK ? rowmask + (int64_t)si * (L >> 5) : nullptr;
     uint4 nxt = (lane < L) ? __ldg(pp + lane) : make_uint4(1, 0, 0xffffffffu, 0xffffffffu);
     for (int64_t i0 = 0; i0 < L && !ws.err; i0 += 32) {
         uint4 cur = nxt;
         int64_t r = i0 + 32 + lane;
         if (r < L) nxt = __ldg(pp + r);                   // prefetch the next 32 rows
+        const uint32_t live = MASK ? __ldg(rm + (i0 >> 5)) : FULL;
         int n = (int)min((int64_t)32, L - i0);
         for (int j = 0; j < n && !ws.err; ++j) {
+            if (MASK && !((live >> j) & 1u)) continue;    // masked row: head and word stack untouched
             uint64_t M = ((uint64_t)__shfl_sync(FULL, cur.w, j) << 32) | __shfl_sync(FULL, cur.z, j);
             const uint32_t pj = __shfl_sync(FULL, cur.x, j);
             if (pj == 0u) { ws.err = BSW_E_INVALID; break; }     // phase A saw a symbol outside the support (reference: IndexError)
@@ -298,11 +305,11 @@ __global__ void __launch_bounds__(BW * 32) k_push_pairs(bsw_streams sv, int firs
 }
 
 // ---- phase B: pop ----------------------------------------------------------------------------------------------------
-template <int NB>
+template <int NB, bool MASK>
 __global__ void __launch_bounds__(BW * 32) k_pop_coarse(bsw_streams sv, int first, int count, const float *__restrict__ mu,
         int64_t mss, const float *__restrict__ sc, int64_t sss, const double *__restrict__ endp, int64_t ers,
         const uint32_t *__restrict__ coarse, const uint2 *__restrict__ fix, int16_t *__restrict__ sym, int64_t L,
-        int bits, int q) {
+        int bits, int q, const uint32_t *__restrict__ rowmask) {
     const int lane = threadIdx.x & 31;
     const int si = blockIdx.x * BW + (threadIdx.x >> 5);
     if (si >= count) return;
@@ -321,14 +328,17 @@ __global__ void __launch_bounds__(BW * 32) k_pop_coarse(bsw_streams sv, int firs
     float mu_w = 0.f, sc_w = 1.f;
     uint2 fx_w = make_uint2(0, 0);
     int my_sym = 0;
-    // per-row scalars (mu, sigma, argmax, remnant) of a block of 32 rows, loaded one block ahead of their use
+    // per-row scalars (mu, sigma, argmax, remnant, row mask word) of a block of 32 rows, loaded one block ahead of their use
     float mu_nx, sc_nx;
     uint2 fx_nx;
+    const uint32_t *rm = MASK ? rowmask + (int64_t)si * (L >> 5) : nullptr;
+    uint32_t live_w = FULL, live_nx;
     {
         int64_t r = ((L - 1) & ~(int64_t)31) + lane;
         mu_nx = r < L ? mub[r] : 0.f;
         sc_nx = r < L ? scb[r] : 1.f;
         fx_nx = r < L ? __ldg(fb + r) : make_uint2(0, 0);
+        live_nx = MASK ? __ldg(rm + ((L - 1) >> 5)) : FULL;
     }
     // coarse cdf rows are independent of the head: keep the loads two rows ahead of their use.  (They are issued AFTER
     // the per-row shuffles below: the first version issued the load first and ncu showed every row stalling ~700 cycles
@@ -338,7 +348,7 @@ __global__ void __launch_bounds__(BW * 32) k_pop_coarse(bsw_streams sv, int firs
     for (int64_t i = L - 1; i >= 0; --i) {
         const int j32 = (int)(i & 31);
         const bool new_block = (j32 == 31 || i == L - 1);
-        if (new_block) { mu_w = mu_nx; sc_w = sc_nx; fx_w = fx_nx; }
+        if (new_block) { mu_w = mu_nx; sc_w = sc_nx; fx_w = fx_nx; live_w = live_nx; }
         const double m_ = (double)__shfl_sync(FULL, mu_w, j32), s_ = (double)__shfl_sync(FULL, sc_w, j32);
         const int bi = (int)__shfl_sync(FULL, fx_w.x, j32);
         const uint32_t rem = __shfl_sync(FULL, fx_w.y, j32);
@@ -347,10 +357,18 @@ __global__ void __launch_bounds__(BW * 32) k_pop_coarse(bsw_streams sv, int firs
             mu_nx = r >= 0 ? mub[r] : 0.f;
             sc_nx = r >= 0 ? scb[r] : 1.f;
             fx_nx = r >= 0 ? __ldg(fb + r) : make_uint2(0, 0);
+            if (MASK && i >= 32) live_nx = __ldg(rm + (i >> 5) - 1);
         }
         const uint32_t base = base_n1;
         base_n1 = base_n2;
         if (i > 1) base_n2 = (lane < NB) ? __ldg(cb + (i - 2) * NB + lane) : 0xffffffffu;
+        if (MASK && !((live_w >> j32) & 1u)) {            // masked row: nothing decoded, the symbol slot keeps what it held
+            if (j32 == 0) {
+                const int64_t r = i + lane;
+                if (r < L) sy[r] = (int16_t)my_sym;
+            }
+            continue;
+        }
         const double rs = __ddiv_rn(1.0, s_);
         const uint32_t mm = (uint32_t)ws.x & mask;                                       // cifar_compress.py:60
         const int chunk = 31 - __clz(__ballot_sync(FULL, base <= mm));                   // base of lanes >= NB is UINT_MAX
@@ -456,7 +474,7 @@ int launch_pop_full(bsw_streams *s, int first, int count, const uint32_t *pfull,
 template <int NB>
 int launch_rows(int phase, bool pop, bsw_streams *s, int first, int count, const float *mu, int64_t mss, const float *sc,
                 int64_t sss, const double *endp, int64_t ers, int16_t *sym, int64_t L, int bits, int q, void *scratch,
-                cudaStream_t st) {
+                const uint32_t *rowmask, cudaStream_t st) {
     dim3 grid((unsigned)L, (count + RW - 1) / RW);
     // pop scratch layout: [coarse: count*L*NB u32, rounded up to 8 bytes] [fix: count*L uint2]
     uint4 *pairs = (uint4 *)scratch;
@@ -468,7 +486,8 @@ int launch_rows(int phase, bool pop, bsw_streams *s, int first, int count, const
     const bool exact = bits > 31 || env_exact;
     BSW_MAX_SHARED_ONCE((k_rows<NB, true, false>)); BSW_MAX_SHARED_ONCE((k_rows<NB, true, true>));
     BSW_MAX_SHARED_ONCE((k_rows<NB, false, false>)); BSW_MAX_SHARED_ONCE((k_rows<NB, false, true>));
-    BSW_MAX_SHARED_ONCE(k_pop_coarse<NB>); BSW_MAX_SHARED_ONCE(k_push_pairs);
+    BSW_MAX_SHARED_ONCE((k_pop_coarse<NB, false>)); BSW_MAX_SHARED_ONCE((k_pop_coarse<NB, true>));
+    BSW_MAX_SHARED_ONCE(k_push_pairs<false>); BSW_MAX_SHARED_ONCE(k_push_pairs<true>);
     if (phase == 0) {
         if (pop) {
             if (exact) k_rows<NB, true, false><<<grid, RW * 32, 0, st>>>(count, L, mu, mss, sc, sss, endp, ers, nullptr, bits, q, nullptr, coarse, fix, kp);
@@ -478,16 +497,21 @@ int launch_rows(int phase, bool pop, bsw_streams *s, int first, int count, const
             else k_rows<NB, false, true><<<grid, RW * 32, 0, st>>>(count, L, mu, mss, sc, sss, endp, ers, sym, bits, q, pairs, nullptr, nullptr, kp);
         }
     } else {
-        if (pop) k_pop_coarse<NB><<<(count + BW - 1) / BW, BW * 32, 0, st>>>(*s, first, count, mu, mss, sc, sss, endp, ers, coarse, fix, sym, L, bits, q);
-        else k_push_pairs<<<(count + BW - 1) / BW, BW * 32, 0, st>>>(*s, first, count, pairs, L, bits);
+        const unsigned g = (count + BW - 1) / BW;
+        if (pop && rowmask) k_pop_coarse<NB, true><<<g, BW * 32, 0, st>>>(*s, first, count, mu, mss, sc, sss, endp, ers, coarse, fix, sym, L, bits, q, rowmask);
+        else if (pop) k_pop_coarse<NB, false><<<g, BW * 32, 0, st>>>(*s, first, count, mu, mss, sc, sss, endp, ers, coarse, fix, sym, L, bits, q, nullptr);
+        else if (rowmask) k_push_pairs<true><<<g, BW * 32, 0, st>>>(*s, first, count, pairs, L, bits, rowmask);
+        else k_push_pairs<false><<<g, BW * 32, 0, st>>>(*s, first, count, pairs, L, bits, nullptr);
     }
     BSW_LAUNCH_CHECK();
     return BSW_OK;
 }
 
-int launch_push_pairs(bsw_streams *s, int first, int count, const void *scratch, int64_t L, int bits, cudaStream_t st) {
-    BSW_MAX_SHARED_ONCE(k_push_pairs);
-    k_push_pairs<<<(count + BW - 1) / BW, BW * 32, 0, st>>>(*s, first, count, (const uint4 *)scratch, L, bits);
+int launch_push_pairs(bsw_streams *s, int first, int count, const void *scratch, int64_t L, int bits, const uint32_t *rowmask,
+                      cudaStream_t st) {
+    BSW_MAX_SHARED_ONCE(k_push_pairs<false>); BSW_MAX_SHARED_ONCE(k_push_pairs<true>);
+    if (rowmask) k_push_pairs<true><<<(count + BW - 1) / BW, BW * 32, 0, st>>>(*s, first, count, (const uint4 *)scratch, L, bits, rowmask);
+    else k_push_pairs<false><<<(count + BW - 1) / BW, BW * 32, 0, st>>>(*s, first, count, (const uint4 *)scratch, L, bits, nullptr);
     BSW_LAUNCH_CHECK();
     return BSW_OK;
 }
@@ -527,7 +551,7 @@ int bsw_pop_shared_table(bsw_streams *s, int first, int count, const uint32_t *P
 int bsw_rows6_build_meta(const double *endp, int64_t ers, int64_t L, int S, void *meta_dev, int *n_affine_host, cudaStream_t st);
 int bsw_rows6_launch(int phase, bool pop, bsw_streams *s, int first, int count, const float *mu, int64_t mss, const float *sc,
                      int64_t sss, const double *endp, int64_t ers, const void *meta, int16_t *sym, int64_t L, int S, int bits,
-                     int q, void *scratch, size_t scratch_bytes, cudaStream_t st);
+                     int q, void *scratch, size_t scratch_bytes, const uint32_t *rowmask, cudaStream_t st);
 
 // Scratch bytes of the two-phase coder for `count` streams of L rows: per row 16 B (push: P, C, reciprocal) or
 // 136 B (pop: 32 chunk bases + argmax/remnant), whichever kernel family runs.
@@ -537,25 +561,29 @@ size_t bsw_rows_scratch_bytes(int count, int64_t L) { return (size_t)count * L *
 // phase 0 = the parallel row-table kernel, phase 1 = the serial coder; call both, in order, on one stream, with the
 // same scratch.  meta != NULL selects the affine-row kernels of ans_rows6.cu (meta = bsw_rows6_build_meta of these
 // endpoint rows); meta == NULL the generic ones above.
+// rowmask (NULL = every row): L/32 words per stream; a clear bit (i & 31) of word i/32 makes the serial phase skip row i --
+// the push leaves the state as it is, the pop decodes nothing there and may leave anything in that symbol slot.  Phase A
+// still builds the masked rows' tables.
 int bsw_logistic_2p(int phase, bool pop, bsw_streams *s, int first, int count, const float *mu, int64_t mss, const float *sc,
                     int64_t sss, const double *endp, int64_t ers, const void *meta, int16_t *sym, int64_t L, int S, int bits,
-                    int q, void *scratch, size_t scratch_bytes, cudaStream_t st) {
+                    int q, void *scratch, size_t scratch_bytes, const uint32_t *rowmask, cudaStream_t st) {
     BSW_REQUIRE(s && first >= 0 && count > 0 && first + count <= s->B, "stream range out of bounds");
     BSW_REQUIRE(mu && sc && endp && sym && scratch && L > 0 && L < 65536 * 32, "two-phase coder: bad arguments");
     BSW_REQUIRE(ers == 0 || ers >= S, "two-phase coder: endpoint rows must hold S doubles (+1e300 padded)");
     BSW_REQUIRE(scratch_bytes >= (pop ? bsw_rows_scratch_bytes(count, L) : (size_t)count * L * 16), "two-phase coder: scratch too small");
     BSW_REQUIRE((((uintptr_t)scratch) & 15) == 0, "two-phase coder: scratch must be 16-byte aligned");
+    BSW_REQUIRE(!rowmask || (L & 31) == 0, "two-phase coder: a row mask needs a multiple of 32 rows");
     if (meta) {
-        if (phase == 1 && !pop) return launch_push_pairs(s, first, count, scratch, L, bits, st);
-        return bsw_rows6_launch(phase, pop, s, first, count, mu, mss, sc, sss, endp, ers, meta, sym, L, S, bits, q, scratch, scratch_bytes, st);
+        if (phase == 1 && !pop) return launch_push_pairs(s, first, count, scratch, L, bits, rowmask, st);
+        return bsw_rows6_launch(phase, pop, s, first, count, mu, mss, sc, sss, endp, ers, meta, sym, L, S, bits, q, scratch, scratch_bytes, rowmask, st);
     }
     switch (S) {
-        case 32:   return launch_rows<1>(phase, pop, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, scratch, st);
-        case 64:   return launch_rows<2>(phase, pop, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, scratch, st);
-        case 128:  return launch_rows<4>(phase, pop, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, scratch, st);
-        case 256:  return launch_rows<8>(phase, pop, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, scratch, st);
-        case 512:  return launch_rows<16>(phase, pop, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, scratch, st);
-        case 1024: return launch_rows<32>(phase, pop, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, scratch, st);
+        case 32:   return launch_rows<1>(phase, pop, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, scratch, rowmask, st);
+        case 64:   return launch_rows<2>(phase, pop, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, scratch, rowmask, st);
+        case 128:  return launch_rows<4>(phase, pop, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, scratch, rowmask, st);
+        case 256:  return launch_rows<8>(phase, pop, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, scratch, rowmask, st);
+        case 512:  return launch_rows<16>(phase, pop, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, scratch, rowmask, st);
+        case 1024: return launch_rows<32>(phase, pop, s, first, count, mu, mss, sc, sss, endp, ers, sym, L, bits, q, scratch, rowmask, st);
     }
     bsw_set_error("two-phase coder: support must be one of 32,64,...,1024 (got %d)", S);
     return BSW_E_INVALID;
@@ -703,8 +731,8 @@ static int abi_2p(bool pop, bsw_streams *s, int first, int count, const float *m
         if (mode == 1 || n_aff == (ers == 0 ? 1 : (int)L)) meta = m;
     }
     const size_t sb = bsw_rows_scratch_bytes(count, L);
-    if (int rc = bsw_logistic_2p(0, pop, s, first, count, mu, mss, sc, sss, endp, ers, meta, sym, L, S, bits, q, scratch, sb, st)) return rc;
-    return bsw_logistic_2p(1, pop, s, first, count, mu, mss, sc, sss, endp, ers, meta, sym, L, S, bits, q, scratch, sb, st);
+    if (int rc = bsw_logistic_2p(0, pop, s, first, count, mu, mss, sc, sss, endp, ers, meta, sym, L, S, bits, q, scratch, sb, nullptr, st)) return rc;
+    return bsw_logistic_2p(1, pop, s, first, count, mu, mss, sc, sss, endp, ers, meta, sym, L, S, bits, q, scratch, sb, nullptr, st);
 }
 extern "C" int bsw_logistic_push_2p(bsw_streams *s, int first, int count, const float *mu, int64_t mss, const float *sc, int64_t sss,
                                     const double *endp, int64_t ers, const int16_t *sym, int64_t L, int S, int bits, int q,

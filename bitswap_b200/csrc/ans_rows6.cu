@@ -324,10 +324,11 @@ __device__ __forceinline__ double shfl_d(double v, int src) {
     return __hiloint2double(__shfl_sync(FULL, __double2hiint(v), src), __shfl_sync(FULL, __double2loint(v), src));
 }
 
+template <bool MASK>          // MASK: skip the rows whose rowmask bit is clear (a template flag, so the unmasked loop is untouched)
 __global__ void __launch_bounds__(PW6 * 32) k_pop6(bsw_streams sv, int first, int count, const float *__restrict__ mu, int64_t mss,
         const float *__restrict__ sc, int64_t sss, const double *__restrict__ endp, int64_t ers,
         const R6RowMeta *__restrict__ meta, int64_t mrs, const uint32_t *__restrict__ bases, const uint2 *__restrict__ fix,
-        int16_t *__restrict__ sym, int64_t L, int S, int bits, int q) {
+        int16_t *__restrict__ sym, int64_t L, int S, int bits, int q, const uint32_t *__restrict__ rowmask) {
     const int lane = threadIdx.x & 31;
     const int si = blockIdx.x * PW6 + (threadIdx.x >> 5);
     if (si >= count) return;
@@ -344,12 +345,15 @@ __global__ void __launch_bounds__(PW6 * 32) k_pop6(bsw_streams sv, int first, in
     const uint32_t mask = (uint32_t)(((uint64_t)1 << bits) - 1);
 
     // per-row scalars of a block of 32 rows (lane j <-> row blk*32 + j), loaded one block ahead of their use; the
-    // float64 plan of each row (t0, dt, window) is then computed by its lane, 32 rows in parallel
+    // float64 plan of each row (t0, dt, window) is then computed by its lane, 32 rows in parallel.  The block's row mask
+    // word (rowmask: L/32 words per stream, NULL = every row) comes with them: a clear bit skips the row.
     float mu_w = 0.f, sc_w = 1.f, mu_nx, sc_nx;
     uint2 fx_w = make_uint2(0, 0), fx_nx;
     double a_nx, d_nx, dev_nx;
     double t0_w = 0.0, dt_w = 1.0, rs_w = 1.0, magic_w = 0.0;
     uint32_t dmask_w = 0;
+    const uint32_t *rm = MASK ? rowmask + (int64_t)si * (L >> 5) : nullptr;
+    uint32_t live_w = FULL, live_nx = FULL;
     auto load_block = [&](int64_t r0) {
         const int64_t r = r0 + lane;
         const bool ok = r >= 0 && r < L;
@@ -358,9 +362,10 @@ __global__ void __launch_bounds__(PW6 * 32) k_pop6(bsw_streams sv, int first, in
         fx_nx = ok ? __ldg(fb + r) : make_uint2(0, 0);
         const R6RowMeta *mp = meta + (ok ? r : 0) * mrs;
         a_nx = __ldg(&mp->a); d_nx = __ldg(&mp->d); dev_nx = __ldg(&mp->dev);
+        if (MASK && r0 >= 0) live_nx = __ldg(rm + (r0 >> 5));
     };
     auto adopt_block = [&]() {
-        mu_w = mu_nx; sc_w = sc_nx; fx_w = fx_nx;
+        mu_w = mu_nx; sc_w = sc_nx; fx_w = fx_nx; live_w = live_nx;
         rs_w = __ddiv_rn(1.0, (double)sc_w);
         R6RowMeta M;
         M.a = a_nx; M.d = d_nx; M.dev = dev_nx; M.rsv = 0.0;
@@ -383,6 +388,13 @@ __global__ void __launch_bounds__(PW6 * 32) k_pop6(bsw_streams sv, int first, in
         const uint32_t base = base_n1;
         base_n1 = base_n2;
         if (i > 1) base_n2 = __ldg(bb + (i - 2) * 32 + lane);
+        if (MASK && !((live_w >> j32) & 1u)) {            // masked row: nothing decoded, the symbol slot keeps what it held
+            if (j32 == 0) {
+                const int64_t r = i + lane;
+                if (r < L) sy[r] = (int16_t)my_sym;
+            }
+            continue;
+        }
         const uint32_t mm = (uint32_t)ws.x & mask;                                       // cifar_compress.py:60
         const uint32_t Ckh = (1u << bits) - (uint32_t)(S - kh);                          // integer cdf at bin kh (dead bins: P = 1)
         uint32_t ps, cs;
@@ -458,7 +470,7 @@ size_t bsw_rows6_scratch_bytes(int count, int64_t L) {
 
 int bsw_rows6_launch(int phase, bool pop, bsw_streams *s, int first, int count, const float *mu, int64_t mss, const float *sc,
                      int64_t sss, const double *endp, int64_t ers, const void *meta, int16_t *sym, int64_t L, int S, int bits,
-                     int q, void *scratch, size_t scratch_bytes, cudaStream_t st) {
+                     int q, void *scratch, size_t scratch_bytes, const uint32_t *rowmask, cudaStream_t st) {
     BSW_REQUIRE(S >= 8 && S <= 1024 && (S & 3) == 0, "affine coder: support must be a multiple of 4 in [8, 1024]");
     BSW_REQUIRE(bits >= 8 && bits <= 31 && q >= 0 && q < bits, "affine coder: bits/quantbits out of range");
     BSW_REQUIRE(scratch_bytes >= (pop ? bsw_rows6_scratch_bytes(count, L) : (size_t)count * L * 16), "affine coder: scratch too small");
@@ -490,8 +502,9 @@ int bsw_rows6_launch(int phase, bool pop, bsw_streams *s, int first, int count, 
 #undef R6_LAUNCH
     } else {
         BSW_REQUIRE(pop, "affine coder: phase B of a push is k_push_pairs");
-        BSW_MAX_SHARED_ONCE(k_pop6);
-        k_pop6<<<(count + PW6 - 1) / PW6, PW6 * 32, 0, st>>>(*s, first, count, mu, mss, sc, sss, endp, ers, mt, mrs, bases, fix, sym, L, S, bits, q);
+        BSW_MAX_SHARED_ONCE(k_pop6<false>); BSW_MAX_SHARED_ONCE(k_pop6<true>);
+        if (rowmask) k_pop6<true><<<(count + PW6 - 1) / PW6, PW6 * 32, 0, st>>>(*s, first, count, mu, mss, sc, sss, endp, ers, mt, mrs, bases, fix, sym, L, S, bits, q, rowmask);
+        else k_pop6<false><<<(count + PW6 - 1) / PW6, PW6 * 32, 0, st>>>(*s, first, count, mu, mss, sc, sss, endp, ers, mt, mrs, bases, fix, sym, L, S, bits, q, nullptr);
     }
     BSW_LAUNCH_CHECK();
     return BSW_OK;

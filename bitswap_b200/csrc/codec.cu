@@ -19,6 +19,7 @@ struct bsw_codec {
     float *mu2, *scale2;                // second mu/sigma pair: in overlap mode infer() and generate() results are alive at once
     int16_t *sym[2];                    // ping-pong latent symbols [max_batch, zdim]
     int16_t *xsym;                      // [max_batch, xdim] pixels as int16 symbols
+    uint32_t *rowmask;                  // [max_batch, xdim / 32] pixel rows a partial block codes (bsw_codec_encode_ext)
     std::vector<int16_t *> zs;          // BB-ANS: all nz latents
     void *scratch;                      // two-phase coder: pairs / coarse cdf of one level
     size_t scratch_bytes;
@@ -53,7 +54,10 @@ int bsw_pop_shared_table(bsw_streams *s, int first, int count, const uint32_t *P
                          int16_t *sym, int64_t L, int S, int bits, cudaStream_t st);
 int bsw_logistic_2p(int phase, bool pop, bsw_streams *s, int first, int count, const float *mu, int64_t mss, const float *sc,
                     int64_t sss, const double *endp, int64_t ers, const void *meta, int16_t *sym, int64_t L, int S, int bits, int q,
-                    void *scratch, size_t scratch_bytes, cudaStream_t st);
+                    void *scratch, size_t scratch_bytes, const uint32_t *rowmask, cudaStream_t st);
+int bsw_logistic_fused(bool pop, bsw_streams *s, int first, int count, const float *mu, int64_t mss, const float *sc,
+                       int64_t sss, const double *endp, int64_t ers, int16_t *sym, int64_t L, int S, int bits, int q,
+                       const uint32_t *rowmask, cudaStream_t st);
 
 __global__ void k_u8_to_i16(const uint8_t *__restrict__ in, int16_t *__restrict__ out, int64_t n) {
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -62,6 +66,47 @@ __global__ void k_u8_to_i16(const uint8_t *__restrict__ in, int16_t *__restrict_
 __global__ void k_i16_to_u8(const int16_t *__restrict__ in, uint8_t *__restrict__ out, int64_t n) {
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = (uint8_t)in[i];
+}
+
+// ---- partial blocks: extents [count][2] = (valid_rows, valid_cols) of each stream's 32x32 block, each in [1, 32] ----------
+// Pixel p of a CHW block (c = p >> 10, y = (p >> 5) & 31, x = p & 31) is valid iff y < valid_rows && x < valid_cols.  The
+// masked pixels are not coded; they hold the edge-replicate fill x[c][min(y, vr-1)][min(x, vc-1)] on both sides, so that
+// the inference net sees the same block when the encoder reads it and when the decoder rebuilds it.
+__device__ __forceinline__ int ext_clamp(int v) { return v < 1 ? 1 : (v > 32 ? 32 : v); }
+// position the fill copies pixel p from (p itself when it is valid); out-of-range extents are clamped here only to keep
+// the read in bounds -- k_rowmask has already flagged that stream, and no coder kernel touches it again
+__device__ __forceinline__ int fill_src(int p, int vr, int vc) {
+    const int y = (p >> 5) & 31, x = p & 31;
+    return (p & ~1023) | (min(y, ext_clamp(vr) - 1) << 5) | min(x, ext_clamp(vc) - 1);
+}
+// One word per (stream, channel, image row): word k of a stream holds the 32 pixels of row k & 31 of channel k >> 5, i.e.
+// exactly the pixel-level rows [32k, 32k + 32) the serial coder kernels walk.  An extent outside [1, 32] flags the stream
+// BSW_E_INVALID (the first failure of a stream is the one kept) and every later coder kernel skips it.
+__global__ void k_rowmask(const int32_t *__restrict__ ext, int64_t n, int wps, uint32_t *__restrict__ mask,
+                          int32_t *__restrict__ flags) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int si = (int)(i / wps), k = (int)(i - (int64_t)si * wps);
+    const int vr = ext[2 * si], vc = ext[2 * si + 1];
+    const bool ok = vr >= 1 && vr <= 32 && vc >= 1 && vc <= 32;
+    mask[i] = (ok && (k & 31) < vr) ? (vc == 32 ? 0xffffffffu : (1u << vc) - 1u) : 0u;
+    if (!ok && k == 0 && flags[si] == BSW_OK) flags[si] = BSW_E_INVALID;
+}
+// encode: uint8 -> int16 symbols with the fill applied on the way
+__global__ void k_u8_to_i16_fill(const uint8_t *__restrict__ in, int16_t *__restrict__ out, int64_t n, int xdim,
+                                 const int32_t *__restrict__ ext) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int si = (int)(i / xdim), p = (int)(i - (int64_t)si * xdim);
+    out[i] = in[(int64_t)si * xdim + fill_src(p, ext[2 * si], ext[2 * si + 1])];
+}
+// decode: the fill in place on the popped symbols -- reads valid positions only, writes masked positions only
+__global__ void k_fill_x(int16_t *__restrict__ x, int64_t n, int xdim, const int32_t *__restrict__ ext) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int si = (int)(i / xdim), p = (int)(i - (int64_t)si * xdim);
+    const int src = fill_src(p, ext[2 * si], ext[2 * si + 1]);
+    if (src != p) x[i] = x[(int64_t)si * xdim + src];
 }
 
 extern "C" int bsw_codec_create(bsw_codec **out, bsw_model *m, bsw_bins *b, int max_batch) {
@@ -81,6 +126,12 @@ extern "C" int bsw_codec_create(bsw_codec **out, bsw_model *m, bsw_bins *b, int 
     BSW_CUDA(cudaMalloc(&c->sym[0], sizeof(int16_t) * c->zdim * max_batch));
     BSW_CUDA(cudaMalloc(&c->sym[1], sizeof(int16_t) * c->zdim * max_batch));
     BSW_CUDA(cudaMalloc(&c->xsym, sizeof(int16_t) * c->xdim * max_batch));
+    BSW_CUDA(cudaMalloc(&c->rowmask, sizeof(uint32_t) * (c->xdim / 32) * max_batch));
+    // symbol buffers start as valid symbols (0): a stream that is skipped because of its error flag leaves them as they
+    // are, and the centre gathers index tables with them
+    BSW_CUDA(cudaMemset(c->sym[0], 0, sizeof(int16_t) * c->zdim * max_batch));
+    BSW_CUDA(cudaMemset(c->sym[1], 0, sizeof(int16_t) * c->zdim * max_batch));
+    BSW_CUDA(cudaMemset(c->xsym, 0, sizeof(int16_t) * c->xdim * max_batch));
     c->zs.assign(c->nz, nullptr);
     {
         size_t a = bsw_rows_scratch_bytes(max_batch, c->zdim), b2 = bsw_rows_scratch_bytes(max_batch, c->xdim);
@@ -125,7 +176,7 @@ extern "C" int bsw_codec_create(bsw_codec **out, bsw_model *m, bsw_bins *b, int 
 extern "C" int bsw_codec_destroy(bsw_codec *c) {
     if (!c) return BSW_OK;
     cudaFree(c->given); cudaFree(c->mu); cudaFree(c->scale); cudaFree(c->mu2); cudaFree(c->scale2); cudaFree(c->scratch_push);
-    cudaFree(c->sym[0]); cudaFree(c->sym[1]); cudaFree(c->xsym);
+    cudaFree(c->sym[0]); cudaFree(c->sym[1]); cudaFree(c->xsym); cudaFree(c->rowmask);
     for (auto p : c->zs) cudaFree(p);
     cudaFree(c->priorP); cudaFree(c->priorC); cudaFree(c->scratch); cudaFree(c->priorCoarse); cudaFree(c->priorFix);
     for (cudaStream_t st : {c->st_conv, c->st_rows, c->st_ser}) if (st) cudaStreamDestroy(st);
@@ -171,6 +222,8 @@ struct Ctx {
     cudaStream_t conv, rows, ser;
     cudaStream_t caller = nullptr;
     int nl = 0;
+    const int32_t *ext = nullptr;       // partial blocks: extents [count][2] on the device (NULL: whole blocks)
+    const uint32_t *xmask = nullptr;    // ... and the pixel-level row mask built from them
     void begin(cudaStream_t user) {
         caller = user;
         if (c->dual_stream) {
@@ -215,6 +268,32 @@ struct Ctx {
         return rc;
     }
     int gather_x16(const int16_t *x);
+    // net input of infer(0) on the encode side: the pixels as given, or for partial blocks the filled symbols
+    int gather_x_in(const uint8_t *x) {
+        if (!ext) return gather_x(x);
+        hop(rows, conv);                                  // (the fill is enqueued on the rows stream)
+        return gather_x16(c->xsym);
+    }
+    // the row mask of the pixel level, on `st` (the stream of the first coder kernel that reads the flags it sets)
+    int build_mask(cudaStream_t st) {
+        const int wps = c->xdim / 32;
+        const int64_t n = (int64_t)count * wps;
+        k_rowmask<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(ext, n, wps, c->rowmask, s->flags + first);
+        BSW_LAUNCH_CHECK();
+        ++nl;
+        xmask = c->rowmask;
+        return BSW_OK;
+    }
+    // decode: the fill on the popped pixel symbols, on the serial stream right after the pop (the hop ser -> conv that
+    // follows the pop orders it before the gather that reads them)
+    int fill_x() {
+        if (!ext) return BSW_OK;
+        const int64_t n = (int64_t)count * c->xdim;
+        k_fill_x<<<(unsigned)((n + 255) / 256), 256, 0, ser>>>(c->xsym, n, c->xdim, ext);
+        BSW_LAUNCH_CHECK();
+        ++nl;
+        return BSW_OK;
+    }
     int gather_z(int lvl, const int16_t *sym) {
         ++nl;
         c->prof.begin(CAT_MISC, conv);
@@ -236,12 +315,12 @@ struct Ctx {
         const int64_t sss = x ? (c->m->d.cond_xscale ? c->xdim : 0) : c->zdim;
         const int cat_rows = x ? CAT_ROWS_X : CAT_ROWS_Z;
         const int cat_ser = x ? (pop ? CAT_POP_X : CAT_PUSH_X) : (pop ? CAT_POP_Z : CAT_PUSH_Z);
+        const uint32_t *rm = x ? xmask : nullptr;
         if (!c->two_phase) {
             hop(rows, ser);
             ++nl;
             c->prof.begin(cat_ser, ser);
-            int rc = pop ? bsw_logistic_pop(s, first, count, mu, L, sc, sss, endp, ers, sym, L, S, 31, q, ser)
-                         : bsw_logistic_push(s, first, count, mu, L, sc, sss, endp, ers, sym, L, S, 31, q, ser);
+            int rc = bsw_logistic_fused(pop, s, first, count, mu, L, sc, sss, endp, ers, sym, L, S, 31, q, rm, ser);
             c->prof.end(ser);
             return rc;
         }
@@ -251,12 +330,12 @@ struct Ctx {
         const size_t scr_bytes = (!pop && c->dual_stream) ? c->scratch_push_bytes : c->scratch_bytes;
         nl += 2;
         c->prof.begin(cat_rows, rows);
-        int rc = bsw_logistic_2p(0, pop, s, first, count, mu, L, sc, sss, endp, ers, meta, sym, L, S, 31, q, scr, scr_bytes, rows);
+        int rc = bsw_logistic_2p(0, pop, s, first, count, mu, L, sc, sss, endp, ers, meta, sym, L, S, 31, q, scr, scr_bytes, rm, rows);
         c->prof.end(rows);
         if (rc) return rc;
         hop(rows, ser);
         c->prof.begin(cat_ser, ser);
-        rc = bsw_logistic_2p(1, pop, s, first, count, mu, L, sc, sss, endp, ers, meta, sym, L, S, 31, q, scr, scr_bytes, ser);
+        rc = bsw_logistic_2p(1, pop, s, first, count, mu, L, sc, sss, endp, ers, meta, sym, L, S, 31, q, scr, scr_bytes, rm, ser);
         c->prof.end(ser);
         return rc;
     }
@@ -298,7 +377,14 @@ static int codec_args_ok(bsw_codec *c, bsw_streams *s, int first, int count, con
 }
 static int ensure_zs(bsw_codec *c) {
     for (auto &p : c->zs)
-        if (!p) BSW_CUDA(cudaMalloc(&p, sizeof(int16_t) * c->zdim * c->max_batch));
+        if (!p) {
+            BSW_CUDA(cudaMalloc(&p, sizeof(int16_t) * c->zdim * c->max_batch));
+            BSW_CUDA(cudaMemset(p, 0, sizeof(int16_t) * c->zdim * c->max_batch));
+        }
+    return BSW_OK;
+}
+static int codec_ext_ok(bsw_codec *c, const int32_t *ext) {
+    BSW_REQUIRE(!ext || c->xdim % 1024 == 0, "bsw_codec: extents need 32x32 pixel blocks");
     return BSW_OK;
 }
 
@@ -310,20 +396,30 @@ static int ensure_zs(bsw_codec *c) {
 // back to back while the float64 table kernels of the push run beside infer(zi+1) on the rows stream: tensor-pipe work
 // and FP64-pipe work of ONE chain share the SMs (the persistent conv kernel leaves room for a table CTA on every SM).
 // Buffers that make this legal: separate (mu, sigma) for the two nets, separate scratch for the push rows.
-extern "C" int bsw_codec_encode(bsw_codec *c, bsw_streams *s, int first, int count, const uint8_t *x, int scheme, void *stream) {
+// extent (may be NULL): partial blocks, see k_rowmask.  The masked pixels are overwritten by the fill before infer(0) sees
+// the block, and the x-level push codes only the valid rows.
+extern "C" int bsw_codec_encode_ext(bsw_codec *c, bsw_streams *s, int first, int count, const uint8_t *x, const int32_t *extent,
+                                    int scheme, void *stream) {
     RC(codec_args_ok(c, s, first, count, x));
+    RC(codec_ext_ok(c, extent));
     Ctx k{c, s, first, count};
+    k.ext = extent;
     k.begin((cudaStream_t)stream);
     const int nz = c->nz;
     int64_t nx = (int64_t)count * c->xdim;
-    k_u8_to_i16<<<(unsigned)((nx + 255) / 256), 256, 0, k.rows>>>(x, c->xsym, nx);       // (read by the push_x table kernel)
+    if (extent) {
+        RC(k.build_mask(k.rows));                        // (the hop rows -> ser before the first pop orders it)
+        k_u8_to_i16_fill<<<(unsigned)((nx + 255) / 256), 256, 0, k.rows>>>(x, c->xsym, nx, c->xdim, extent);
+    } else {
+        k_u8_to_i16<<<(unsigned)((nx + 255) / 256), 256, 0, k.rows>>>(x, c->xsym, nx);   // (read by the push_x table kernel)
+    }
     BSW_LAUNCH_CHECK();
     ++k.nl;
     int16_t *zsym = c->sym[0], *ztop = c->sym[1];
     if (scheme == 0) {
         // Bit-Swap sender (cifar_compress.py:178-204)
         for (int zi = 0; zi < nz; ++zi) {
-            if (zi == 0) RC(k.gather_x(x)); else RC(k.gather_z(zi - 1, zsym));           // :180
+            if (zi == 0) RC(k.gather_x_in(x)); else RC(k.gather_z(zi - 1, zsym));        // :180
             RC(k.net(true, zi));                                                            // :181
             k.hop(k.conv, k.rows);
             RC(k.level(true, zi, true, ztop));                                              // :182-187
@@ -339,7 +435,7 @@ extern "C" int bsw_codec_encode(bsw_codec *c, bsw_streams *s, int first, int cou
         // BB-ANS sender (cifar_compress.py:208-242): all pops first, then all pushes
         RC(ensure_zs(c));
         for (int zi = 0; zi < nz; ++zi) {
-            if (zi == 0) RC(k.gather_x(x)); else RC(k.gather_z(zi - 1, c->zs[zi - 1]));
+            if (zi == 0) RC(k.gather_x_in(x)); else RC(k.gather_z(zi - 1, c->zs[zi - 1]));
             RC(k.net(true, zi));
             k.hop(k.conv, k.rows);
             RC(k.level(true, zi, true, c->zs[zi]));
@@ -360,11 +456,20 @@ extern "C" int bsw_codec_encode(bsw_codec *c, bsw_streams *s, int first, int cou
     c->launches = k.nl;
     return BSW_OK;
 }
+extern "C" int bsw_codec_encode(bsw_codec *c, bsw_streams *s, int first, int count, const uint8_t *x, int scheme, void *stream) {
+    return bsw_codec_encode_ext(c, s, first, count, x, nullptr, scheme, stream);
+}
 
-extern "C" int bsw_codec_decode(bsw_codec *c, bsw_streams *s, int first, int count, uint8_t *x, int scheme, void *stream) {
+// extent (may be NULL): partial blocks.  The x-level pop decodes only the valid rows; right after it the fill rebuilds the
+// masked pixels, so infer(0) sees the encoder's block and the returned block holds the fill there.
+extern "C" int bsw_codec_decode_ext(bsw_codec *c, bsw_streams *s, int first, int count, uint8_t *x, const int32_t *extent,
+                                    int scheme, void *stream) {
     RC(codec_args_ok(c, s, first, count, x));
+    RC(codec_ext_ok(c, extent));
     Ctx k{c, s, first, count};
+    k.ext = extent;
     k.begin((cudaStream_t)stream);
+    if (extent) RC(k.build_mask(k.ser));
     const int nz = c->nz;
     int16_t *ztop = c->sym[0], *sym = c->sym[1];
     if (scheme == 0) {
@@ -376,6 +481,7 @@ extern "C" int bsw_codec_decode(bsw_codec *c, bsw_streams *s, int first, int cou
             RC(k.net(false, zi));                                                           // :297
             k.hop(k.conv, k.rows);
             RC(k.level(true, zi == 0 ? -1 : zi - 1, false, zi == 0 ? c->xsym : sym));       // :298-303
+            if (zi == 0) RC(k.fill_x());
             k.hop(k.ser, k.conv);
             if (zi == 0) RC(k.gather_x16(c->xsym)); else RC(k.gather_z(zi - 1, sym));       // :306
             RC(k.net(true, zi));                                                            // :307
@@ -393,6 +499,7 @@ extern "C" int bsw_codec_decode(bsw_codec *c, bsw_streams *s, int first, int cou
             RC(k.net(false, zi));
             k.hop(k.conv, k.rows);
             RC(k.level(true, zi == 0 ? -1 : zi - 1, false, zi == 0 ? c->xsym : c->zs[zi - 1]));
+            if (zi == 0) RC(k.fill_x());
             k.hop(k.ser, k.conv);
         }
         for (int zi = nz - 1; zi >= 0; --zi) {
@@ -409,4 +516,7 @@ extern "C" int bsw_codec_decode(bsw_codec *c, bsw_streams *s, int first, int cou
     k.end();
     c->launches = k.nl + 1;
     return BSW_OK;
+}
+extern "C" int bsw_codec_decode(bsw_codec *c, bsw_streams *s, int first, int count, uint8_t *x, int scheme, void *stream) {
+    return bsw_codec_decode_ext(c, s, first, count, x, nullptr, scheme, stream);
 }

@@ -291,6 +291,17 @@ int bsw_codec_encode(bsw_codec *c, bsw_streams *s, int first, int count, const u
                      void *stream);
 int bsw_codec_decode(bsw_codec *c, bsw_streams *s, int first, int count, uint8_t *x_dev, int scheme,
                      void *stream);
+/* Partial blocks (the edges of an image that is not a multiple of 32 on a side).  extent_dev int32 [count, 2] =
+ * (valid_rows, valid_cols) of each stream's block, each in [1, 32]; pixel (c, y, x) is valid iff y < valid_rows and
+ * x < valid_cols.  Masked pixels are not coded: both sides overwrite them with the edge-replicate fill
+ * x[c][min(y, valid_rows-1)][min(x, valid_cols-1)] before infer(0) sees the block, the x-level push/pop skip their rows,
+ * and decode returns the fill there.  The latent levels are coded as for a whole block.  An extent outside [1, 32] flags
+ * that stream BSW_E_INVALID; the other streams are unaffected.  extent_dev == NULL is exactly bsw_codec_encode/decode,
+ * and all-(32, 32) extents give bit-identical streams. */
+int bsw_codec_encode_ext(bsw_codec *c, bsw_streams *s, int first, int count, const uint8_t *x_dev,
+                         const int32_t *extent_dev, int scheme, void *stream);
+int bsw_codec_decode_ext(bsw_codec *c, bsw_streams *s, int first, int count, uint8_t *x_dev,
+                         const int32_t *extent_dev, int scheme, void *stream);
 /* Number of kernel launches the last encode/decode call enqueued (bench.py's gpu_launches). */
 int64_t bsw_codec_last_launches(const bsw_codec *c);
 /* Stream placement inside one encode/decode call: 0 (default) = every kernel on the caller's stream; 1 = conv kernels
